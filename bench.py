@@ -2,6 +2,7 @@
 """bench.py — headline benchmark of the B200 visualDet3D hot path (contract: see the task brief / DESIGN.md).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config stereo|gac|monoflex|km3d|yolo3d] [--batch B]
+                    [--dump-outputs DIR]
     torchrun --nproc-per-node N bench.py --gpus N ...        (one rank per GPU, NCCL)
 
 Default workload (= BASELINE.json configs[1] / the `metric`): a "step" = one YOLOStereo3D forward (backbone -> cost volumes -> neck ->
@@ -15,9 +16,12 @@ post-optimisation of its shipped config on, monoflex / km3d = configs[3], yolo3d
                (crop / resize / normalise) -> forward -> all-gather -> D2H of the records; `e2e_f32` = the same with float32 network
                inputs (4x the H2D bytes), the form round 1 reported
   roofline     scale-4 PSMCosine kernel (dominant cost-volume kernel; stereo only): algorithmic bytes / CUDA-event time vs measured HBM peak
-  cpu_baseline / --impl reference : the UNMODIFIED reference (oracle/_ref/visualDet3D or /root/reference, loaded by oracle/refload.py)
+  --dump-outputs DIR : after the timing, DIR/<name>.npy holds what the last timed step of each leg returned (per-image scores, boxes,
+               classes and detection counts; the device leg's record block too): inputs and weights are seeded, so two builds of the project
+               can be compared output for output
+  cpu_baseline / --impl reference : the UNMODIFIED reference (a checkout found by oracle/refload.py, e.g. via $VISUALDET3D_REF)
                running its own PyTorch forward on this host's cores (`kind: "reference"`); falls back to the oracle port (`"port"`)
-               only when no copy of the reference package travelled to this box
+               when no reference checkout is importable on this machine
 """
 from __future__ import annotations
 
@@ -316,7 +320,13 @@ def main():
     ap.add_argument("--batch", type=int, default=None, help="samples per GPU per step (default: 8; yolo3d 1)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--profile-mode", action="store_true", help="device-resident steps only (for ncu): no e2e leg, no CPU baseline")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step of every leg to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.profile_mode or args.impl == "reference"):
+        ap.error("--dump-outputs writes the outputs of the timed B200 legs: not with --profile-mode or --impl reference")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -462,6 +472,7 @@ def main():
         drain()                                   # the last all-gathers are inside the timed region
         e1.record()
         barrier()
+        last_records = (gat_bufs if world > 1 else rec_bufs)[(args.steps - 1) % 2].clone()     # the last timed step's (gathered) records
         launches = _lib.launch_count() + graph_launches() - g0          # kernels launched directly + kernels inside the replayed graphs
         ms_dev = e0.elapsed_time(e1)
         ms_fwd = e0.elapsed_time(e_fwd)
@@ -563,9 +574,25 @@ def main():
                                           "frac_of_hbm_peak": alg[k] / 1e9 / (statistics.mean(v) / 1e3) / peak} for k, v in situ.items() if k in alg and v}
     if not args.no_cpu_baseline and world == 1:          # the CPU arm is timed on rank 0 at N = 1 only (the driver runs --impl reference for every N)
         out["cpu_baseline"] = cpu_baseline_subprocess(args.config, B)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"device": parallel.unpack_records(last_records.cpu()), "e2e": res_u8, "e2e_f32": res_f32}, last_records)
     print(json.dumps(out))
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(dirname: str, legs, records) -> None:
+    """legs: leg name -> per-image (scores, boxes, classes) of the GLOBAL batch; records: the device leg's record block."""
+    import numpy as np
+    import torch
+    os.makedirs(dirname, exist_ok=True)
+    arrays = {"device_records": records.cpu()}
+    for leg, res in legs.items():
+        arrays[f"{leg}_counts"] = torch.tensor([len(s) for s, _, _ in res])
+        for i, what in enumerate(("scores", "boxes", "classes")):
+            arrays[f"{leg}_{what}"] = torch.cat([r[i].cpu() for r in res])
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), a.to(torch.float32).numpy())
 
 
 def E_overflow() -> bool:

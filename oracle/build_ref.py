@@ -31,29 +31,10 @@ def _so_path(name: str) -> str:
     return os.path.join(OUT, name, name + ".so")
 
 
-def copy_package() -> None:
-    """The reference's Python package, copied verbatim next to its compiled extensions (oracle/_ref/visualDet3D, git-ignored, ships to
-    the GPU box with the snapshot): `bench.py --impl reference` then times the REAL reference on the box's host cores and the seam
-    tests run its unmodified modules against the B200 ops.  Nothing under oracle/_ref is ever imported by the product package."""
-    import shutil
-    src, dst = os.path.join(REF, "visualDet3D"), os.path.join(OUT, "visualDet3D")
-    if not os.path.isdir(src):
-        return
-    stamp = os.path.join(dst, ".copied_from")
-    if os.path.exists(stamp):
-        return
-    if os.path.isdir(dst):
-        shutil.rmtree(dst)
-    shutil.copytree(src, dst, ignore=shutil.ignore_patterns("__pycache__", "*.pyc", "*.so", "build", "*.egg-info"))
-    with open(stamp, "w") as f:
-        f.write(src + "\n")
-
-
 def build(verbose: bool = False) -> None:
     """No-op when the reference tree is absent (GPU box) or the outputs are already there."""
     if not os.path.isdir(OPS):
         return
-    copy_package()
     todo = [n for n in SOURCES if not os.path.exists(_so_path(n))]
     if not todo:
         return

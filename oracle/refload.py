@@ -5,12 +5,11 @@
                                           passed in (`visualdet3d_b200.ops.dcn` / `.ops.iou3d` = the drop-in test, or the reference's own
                                           extensions built by oracle/build_ref.py)
 
-Where the package comes from: $VISUALDET3D_REF, else /root/reference (build container, read-only mount), else oracle/_ref (the copy
-`oracle/build_ref.py` ships to the GPU box next to the reference's compiled extensions; git-ignored).  No reference source is edited:
-the recipe of SURVEY.md section 8(c) is environmental shims only (easydict / skimage / matplotlib stand-ins, the numba CUDA simulator,
+Where the package comes from: the reference checkout `oracle/build_ref.py` compiles the extensions from ($VISUALDET3D_REF or its
+default).  No reference source is edited or copied: the recipe of SURVEY.md section 8(c) is environmental shims only (easydict / skimage / matplotlib stand-ins, the numba CUDA simulator,
 and -- CPU mode only -- `Tensor.cuda` as the identity because the reference hard-codes `.cuda()` calls, PSM_cost_volume.py:51,83).
 
-Used by: tests/golden/make_golden*.py (fixture generation), bench.py --impl reference (the CPU arm), tests/test_reference_seam*.py.
+Used by: tests/golden/make_golden*.py (fixture generation), bench.py --impl reference (the CPU arm); `to_edict` by tests/workers/seam_cpu.py.
 """
 import os
 import sys
@@ -20,12 +19,12 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 
 
 def ref_root() -> str:
-    env = os.environ.get("VISUALDET3D_REF")
-    if env:
-        return env
-    if os.path.isdir("/root/reference/visualDet3D"):
-        return "/root/reference"
-    return os.path.join(HERE, "_ref")
+    sys.path.insert(0, HERE)
+    try:
+        import build_ref
+    finally:
+        sys.path.remove(HERE)
+    return build_ref.REF
 
 
 def available() -> bool:
@@ -116,7 +115,7 @@ def load_reference(device: str = "cpu", dcn_ext=None, iou3d_ext=None):
         _install_ext(dcn_ext, iou3d_ext)
     root = ref_root()
     if not os.path.isdir(os.path.join(root, "visualDet3D")):
-        raise FileNotFoundError(f"no reference package under {root} (run oracle/build_ref.py in the build container)")
+        raise FileNotFoundError(f"no reference package under {root} (set VISUALDET3D_REF to a reference checkout)")
     sys.path.insert(0, root)
     import visualDet3D
     import visualDet3D.networks  # registers detectors
